@@ -6,6 +6,7 @@ a batch of 1024 synthetic frames per GPU (64 GiB resident in HBM, >> the 126 MB 
 one pass of the fused thumbnail kernel over the whole batch, frames resident in HBM.
 
   python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1)
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step computed, DIR/*.npy
   python bench.py --impl reference ...                      CPU arm (the oracle port
                                                             of the reference algorithm)
 
@@ -38,6 +39,29 @@ WORKLOAD = "vips_thumbnail 4K->512 uchar RGBA (premultiply,shrinkv4,reducev13,sh
 WORKLOAD_PIPELINE = ("vips_thumbnail 4K->512 uchar RGBA then vips_sharpen (sRGB->LabS, 3-tap integer blur of L, LUT, LabS->sRGB) on the 512x512 "
                      "result, synthetic frames, device-resident")
 PIPELINE = False  # set by --workload pipeline: the CPU arm and the GPU arm both append the sharpen stage
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(dirname, arrays, budget=DUMP_BYTES):
+    """--dump-outputs: each device array as <dirname>/<name>.npy in float32 (float64 data stays float64).  An array over
+    its share of the budget is sampled along its first axis by a fixed seed, the indices written beside it as
+    <name>_index.npy, so that two builds run with the same arguments write files that compare entry for entry."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    share = budget // len(arrays)
+    for name, t in arrays.items():
+        dt = np.dtype(np.float64 if t.dtype == torch.float64 else np.float32)
+        if t.numel() * dt.itemsize > share:
+            if t[0].numel() * dt.itemsize > share:
+                t = t.reshape(-1)
+            k = max(1, share // (t[0].numel() * dt.itemsize))
+            idx = np.sort(np.random.default_rng(0).choice(t.shape[0], k, replace=False))
+            np.save(os.path.join(dirname, name + "_index.npy"), idx.astype(np.float64))
+            t = t[torch.as_tensor(idx, device=t.device)]
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy().astype(dt))
 
 
 def peaks():
@@ -301,7 +325,7 @@ def side_workload(args):
         dt = time.perf_counter() - t
         return {"value": units / dt, "unit": "Mpixels/s", "cores": 1, "kind": "port", "sample": "%s, %.1f s" % (sample, dt)}
 
-    def run(fn, alg_bytes, label, units, unit_name, cpu=None):
+    def run(fn, alg_bytes, label, units, unit_name, cpu=None, outputs=None):
         for _ in range(args.warmup):
             fn()
         torch.cuda.synchronize()
@@ -312,6 +336,8 @@ def side_workload(args):
             fn()
         e1.record(stream)
         torch.cuda.synchronize()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         ms = e0.elapsed_time(e1) / args.steps
         ach = alg_bytes / (ms / 1e3) / 1e9
         print(json.dumps({"metric": label, "value": units / (ms / 1e3), "unit": unit_name, "n_gpus": 1,
@@ -337,7 +363,7 @@ def side_workload(args):
         from oracle import pyconv
         ca = (np.random.default_rng(1234).random((2048, 2048, 3), dtype=np.float32) * 255)
         cpu = cpu_side(lambda: pyconv.convsep(ca, m, scale, off, "float"), 2048 * 2048 / 1e6, "2048x2048x3 float32")
-        run(fn, 2 * a.numel() * 4, "vips_convsep 15-tap Gaussian float on 8192x8192 RGB float32", n * n / 1e6, "Mpixels/s", cpu)
+        run(fn, 2 * a.numel() * 4, "vips_convsep 15-tap Gaussian float on 8192x8192 RGB float32", n * n / 1e6, "Mpixels/s", cpu, {"out": out})
     elif args.workload == "colour":
         n = 16384
         a = torch.randint(0, 256, (n, n, 3), dtype=torch.uint8, device=dev)
@@ -359,7 +385,7 @@ def side_workload(args):
         cpu = cpu_side(lambda: pyoracle.colourspace(pyoracle.colourspace(ca, "lab", "srgb"), "srgb", "lab"),
                        2 * 2048 * 2048 / 1e6, "2048x2048x3 uint8, both directions")
         run(fn, 2 * (a.numel() + lab.numel() * 4), "vips_colourspace sRGB->Lab->sRGB round trip on 16384x16384",
-            2 * n * n / 1e6, "Mpixels/s", cpu)
+            2 * n * n / 1e6, "Mpixels/s", cpu, {"lab": lab, "srgb": back})
     elif args.workload == "reduce49":
         n = 4096
         a = torch.randint(0, 256, (n, n, 4), dtype=torch.uint8, device=dev)
@@ -374,7 +400,7 @@ def side_workload(args):
         cpu = cpu_side(lambda: pyoracle.reduceh(pyoracle.reducev(ca, 8.0, "lanczos3", 0.0), 8.0, "lanczos3", 0.0),
                        n * n / 1e6, "one 4096x4096 RGBA frame")
         run(fn, a.numel() + out.numel(), "vips_reduce(8, 8) Lanczos3 gap 0 (49 taps) on one 4096x4096 uchar RGBA",
-            n * n / 1e6, "Mpixels/s", cpu)
+            n * n / 1e6, "Mpixels/s", cpu, {"out": out})
     elif args.workload == "upsize":
         # SURVEY 8(a) a7: vips_resize x2 = vips_affine + bicubic (resize.c:235-305)
         n = 4096
@@ -389,7 +415,7 @@ def side_workload(args):
         ca = np.random.default_rng(1234).integers(0, 256, (1024, 1024, 4), dtype=np.uint8)
         cpu = cpu_side(lambda: pyoracle.resize(ca, 2.0), 4 * 1024 * 1024 / 1e6, "1024x1024 RGBA -> 2048x2048")
         run(fn, a.numel() + out.numel(), "vips_resize x2 (affine + bicubic) 4096x4096 uchar RGBA -> 8192x8192",
-            4 * n * n / 1e6, "output Mpixels/s", cpu)
+            4 * n * n / 1e6, "output Mpixels/s", cpu, {"out": out})
     elif args.workload == "sharpen":
         # SURVEY 8(a) a11: vips_sharpen defaults on an sRGB image (sRGB -> LabS, L blur + LUT, LabS -> sRGB)
         n = 4096
@@ -403,7 +429,7 @@ def side_workload(args):
         from oracle import pyconv
         ca = np.random.default_rng(1234).integers(0, 256, (1024, 1024, 3), dtype=np.uint8)
         cpu = cpu_side(lambda: pyconv.sharpen(ca, "srgb"), 1024 * 1024 / 1e6, "1024x1024 RGB")
-        run(fn, 2 * a.numel(), "vips_sharpen defaults on 4096x4096 sRGB uchar", n * n / 1e6, "Mpixels/s", cpu)
+        run(fn, 2 * a.numel(), "vips_sharpen defaults on 4096x4096 sRGB uchar", n * n / 1e6, "Mpixels/s", cpu, {"out": out})
     elif args.workload == "thumbnail_linear":
         # north_star's "fused Lanczos3-reduce -> sRGB -> linear" path: vips_thumbnail_image(linear=TRUE), SURVEY 3.1b
         F = max(1, min(args.frames, 128))
@@ -426,7 +452,7 @@ def side_workload(args):
         ca = np.random.default_rng(7).integers(0, 256, (H, W, BANDS), dtype=np.uint8)
         cpu = cpu_side(lambda: pyoracle.thumbnail_image(ca, TARGET, linear=True), W * H / 1e6, "one 4096x4096 RGBA frame")
         run(fn, plan.bytes_per_frame * F, "vips_thumbnail_image(linear=TRUE) 4K->512 uchar RGBA, %d frames (%s)" % (F, plan.kernel),
-            F * W * H / 1e6, "Mpixels/s", cpu)
+            F * W * H / 1e6, "Mpixels/s", cpu, {"thumbnails": outs})
     elif args.workload == "icc":
         # SURVEY 8(a) a20: vips_icc_import then vips_icc_export through an sRGB-like v4 matrix/TRC profile
         sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -455,7 +481,7 @@ def side_workload(args):
                            "2048x2048x3 uint8 through lcms2 2.18 itself, both directions")
             cpu["kind"] = "reference"
         run(fn, 2 * (a.numel() + lab.numel() * 4), "vips_icc_import + vips_icc_export (sRGB-like v4 profile) on 8192x8192",
-            2 * n * n / 1e6, "Mpixels/s", cpu)
+            2 * n * n / 1e6, "Mpixels/s", cpu, {"lab": lab, "srgb": back})
     elif args.workload in ("rank", "flatten", "greyscale"):
         # SURVEY 8f ranks 3 / 4 (DESIGN 4.10-4.12): parity-green in round 2, never timed there (the GPU budget was spent)
         n = 4096
@@ -471,7 +497,7 @@ def side_workload(args):
                 vb._check(L.vb200_rank(C.byref(cin), C.byref(cout), 3, 3, 4))
             ca = rng.integers(0, 256, (1024, 1024, 3), dtype=np.uint8)
             cpu = cpu_side(lambda: pyconv.median(ca, 3), 1024 * 1024 / 1e6, "1024x1024 RGB")
-            run(fn, 2 * a.numel(), "vips_median 3x3 on 4096x4096 sRGB uchar", n * n / 1e6, "Mpixels/s", cpu)
+            run(fn, 2 * a.numel(), "vips_median 3x3 on 4096x4096 sRGB uchar", n * n / 1e6, "Mpixels/s", cpu, {"out": out})
         elif args.workload == "flatten":
             a = torch.randint(0, 256, (n, n, 4), dtype=torch.uint8, device=dev)
             out = torch.empty((n, n, 3), dtype=torch.uint8, device=dev)
@@ -483,7 +509,8 @@ def side_workload(args):
                 vb._check(L.vb200_flatten(C.byref(cin), C.byref(cout), bg, 3, 0.0))
             ca = rng.integers(0, 256, (1024, 1024, 4), dtype=np.uint8)
             cpu = cpu_side(lambda: pyconv.flatten(ca, (255, 255, 255)), 1024 * 1024 / 1e6, "1024x1024 RGBA")
-            run(fn, a.numel() + out.numel(), "vips_flatten (white background) on 4096x4096 RGBA uchar", n * n / 1e6, "Mpixels/s", cpu)
+            run(fn, a.numel() + out.numel(), "vips_flatten (white background) on 4096x4096 RGBA uchar", n * n / 1e6, "Mpixels/s", cpu,
+                {"out": out})
         else:
             from oracle import pyoracle
             a = torch.randint(0, 256, (n, n, 3), dtype=torch.uint8, device=dev)
@@ -495,7 +522,7 @@ def side_workload(args):
                 vb._check(L.vb200_colourspace(C.byref(cin), C.byref(cout), 1))
             ca = rng.integers(0, 256, (1024, 1024, 3), dtype=np.uint8)
             cpu = cpu_side(lambda: pyoracle.colourspace(ca, "b-w", "srgb"), 1024 * 1024 / 1e6, "1024x1024 RGB")
-            run(fn, a.numel() + out.numel(), "vips_colourspace sRGB -> B_W on 4096x4096 uchar", n * n / 1e6, "Mpixels/s", cpu)
+            run(fn, a.numel() + out.numel(), "vips_colourspace sRGB -> B_W on 4096x4096 uchar", n * n / 1e6, "Mpixels/s", cpu, {"out": out})
     elif args.workload in ("thumbnail_jpeg", "thumbnail_jpeg_norestart", "thumbnail_jpeg_progressive"):
         # SURVEY 8(f) rank 1: vips_thumbnail_buffer() of JPEG streams.  Host memory holds only the COMPRESSED frames; the
         # shrink-on-load decode (thumbnail.c:489-517 picks 1/4 for 4K -> 512) and the thumbnail run on the device.
@@ -559,6 +586,12 @@ def side_workload(args):
             fn()
         torch.cuda.synchronize()
         dt = (time.perf_counter() - t0) / args.steps
+        if args.dump_outputs:
+            dumped = {"thumbnails": outs}
+            if args.save:
+                dumped["jpeg_streams"] = torch.frombuffer(bytearray(b"".join(saved)), dtype=torch.uint8)
+                dumped["jpeg_stream_lengths"] = torch.tensor([len(x) for x in saved], dtype=torch.float64)
+            dump_outputs(args.dump_outputs, dumped)
         cpu = None
         if not args.no_cpu:
             import multiprocessing as mp
@@ -605,6 +638,9 @@ def main():
     ap.add_argument("--alpha", default="random", choices=["random", "opaque"],
                     help="alpha band of the synthetic frames: random (the headline) | opaque (255 everywhere, what a PNG without "
                          "transparency decodes to: the kernel's opaque-stage fast path; a second line, never the headline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float32; outputs over "
+                         "64 MB in all are sampled by a fixed seed, the indices in DIR/<name>_index.npy)")
     ap.add_argument("--workload", default="thumbnail",
                     help="thumbnail (the headline, default) | pipeline (BASELINE config 5: thumbnail + sharpen + sRGB, runs under "
                          "--gpus N like the headline) | thumbnail_jpeg | thumbnail_jpeg_norestart | thumbnail_jpeg_progressive (decode staging, SURVEY 8f; --save adds the encoder) | thumbnail_linear | convsep | colour | reduce49 | upsize | sharpen | icc | rank | flatten | greyscale: the other BASELINE.json "
@@ -614,6 +650,8 @@ def main():
     global PIPELINE
     PIPELINE = args.workload == "pipeline"
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the device computed: not with --impl reference")
         return reference_arm(args)
     if args.workload not in ("thumbnail", "pipeline"):
         return side_workload(args)
@@ -716,6 +754,8 @@ def main():
     barrier()
     ev_mid[:] = []
     launches = vb.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"thumbnails" + ("" if world == 1 else "_rank%d" % rank): outs}, DUMP_BYTES // world)
     clocks = sampler.stop() if rank == 0 else None
     total_ms = evs[0].elapsed_time(evs[-1])
     per_step = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]

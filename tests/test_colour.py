@@ -1,5 +1,5 @@
 """Colour path.  CPU: the oracle against the reference's own line functions
-(oracle/_ref) and the known answers in the reference's test_colour.py.  GPU:
+(oracle/_ref, or its outputs' stored digests: tests/refgold.py) and the known answers in the reference's test_colour.py.  GPU:
 the fused route kernel against the oracle, bit for bit (the spec allows 1 ULP
 on float; we assert 0) through the C ABI.
 """
@@ -8,11 +8,11 @@ import pytest
 
 from oracle import pyoracle as orc
 from oracle import pyref
+from refgold import ref  # noqa: F401
 
 SPACES = ["srgb", "scrgb", "xyz", "lab", "labs", "rgb16"]
 SPACE_DT = {"srgb": np.uint8, "rgb16": np.uint16, "labs": np.int16, "scrgb": np.float32, "xyz": np.float32,
             "lab": np.float32}
-needs_ref = pytest.mark.skipif(not pyref.available(), reason="oracle/_ref not built")
 
 
 def sample(space, rng, n=20000, wild=False):
@@ -45,21 +45,18 @@ STEP_SPACE = [("sRGB2scRGB", "srgb"), ("RGB162scRGB", "rgb16"), ("scRGB2XYZ", "s
               ("scRGB2sRGB", "scrgb"), ("scRGB2RGB16", "scrgb")]
 
 
-@needs_ref
-def test_tables_match_reference():
+def test_tables_match_reference(ref):
     for which in range(5):
-        assert np.array_equal(orc.colour_table(which), pyref.colour_table(which))
+        ref.check(orc.colour_table(which), lambda: pyref.colour_table(which))
 
 
-@needs_ref
 @pytest.mark.parametrize("step,space", STEP_SPACE)
-def test_oracle_step_matches_reference_line(step, space):
+def test_oracle_step_matches_reference_line(ref, step, space):
     rng = np.random.default_rng(7)
     for wild in (False, True):
         a = sample(space, rng, wild=wild)
-        want = pyref.colour_line(step, a)
         got = orc.colour_step(a.reshape(1, -1, 3), step, space).reshape(-1, 3)
-        assert np.array_equal(want, got, equal_nan=True), step
+        ref.check(got, lambda: pyref.colour_line(step, a), step)
 
 
 def test_known_answer_lab_to_xyz():
@@ -169,14 +166,12 @@ def sample_new(space, rng, n=20000):
     return a
 
 
-@needs_ref
 @pytest.mark.parametrize("step,space", NEW_STEPS)
-def test_oracle_new_converters_match_reference_lines(step, space):
+def test_oracle_new_converters_match_reference_lines(ref, step, space):
     """the reference's own Lab2LCh.c / LCh2Lab.c / XYZ2Yxy.c / Yxy2XYZ.c under oracle/_ref (same glibc: bit for bit)"""
     a = sample_new(space, np.random.default_rng(17))
-    want = pyref.colour_line(step, a)
     got = orc.colour_step(a.reshape(1, -1, 3), step, space).reshape(-1, 3)
-    assert np.array_equal(got, want, equal_nan=True)
+    ref.check(got, lambda: pyref.colour_line(step, a))
 
 
 def test_new_spaces_routes_follow_the_table():
@@ -196,9 +191,8 @@ def test_new_spaces_routes_follow_the_table():
 ALL_SPACES = SPACES + ["lch", "yxy"]
 
 
-@needs_ref
 @pytest.mark.parametrize("bands", [3, 4, 5])
-def test_oracle_colourspace_matches_reference_build(bands):
+def test_oracle_colourspace_matches_reference_build(ref, bands):
     """the whole of vips_colourspace, not only the line functions: colourspace.c's route table and build, a real VipsColour
     object per step (colour.c: extra bands detached, alpha rescaled by the max_alpha ratio through linear.c, cast through
     cast.c and re-attached; the input casts of VipsColourCode / VipsColourTransform), vips_colour_gen pulling tiles --
@@ -211,15 +205,12 @@ def test_oracle_colourspace_matches_reference_build(bands):
             a = np.concatenate([a, sample(base, rng, n=31 * 47)[:, :bands - 3]], axis=1)
         a = a.reshape(31, 47, bands)
         for dst in ALL_SPACES:
-            ref = pyref.RefImage.from_array(a, orc.SPACES[src]).colourspace(dst, src)
-            want = ref.numpy(tile=(16, 8))
             got = orc.colourspace(a, dst, src)
-            assert got.dtype == want.dtype, (src, dst)
-            assert np.array_equal(got, want, equal_nan=True), (src, dst, bands)
+            ref.check(got, lambda: pyref.RefImage.from_array(a, orc.SPACES[src]).colourspace(dst, src).numpy(tile=(16, 8)),
+                      (src, dst, bands))
 
 
-@needs_ref
-def test_oracle_colourspace_wild_floats_and_foreign_formats_match_reference_build():
+def test_oracle_colourspace_wild_floats_and_foreign_formats_match_reference_build(ref):
     """NaN / Inf pixels AND alpha through the reference's builds (alpha: linear.c then cast.c's float -> int clip), and
     images whose band format is not the one their interpretation implies (the reference casts the whole image first:
     colour.c:338-347, 421-428)"""
@@ -231,8 +222,8 @@ def test_oracle_colourspace_wild_floats_and_foreign_formats_match_reference_buil
                 a = np.concatenate([a, sample("lab", rng, n=23 * 40, wild=True)[:, :1]], axis=1)
             a = a.reshape(23, 40, bands)
             for dst in ALL_SPACES:
-                want = pyref.RefImage.from_array(a, orc.SPACES[src]).colourspace(dst, src).numpy()
-                assert np.array_equal(orc.colourspace(a, dst, src), want, equal_nan=True), (src, dst, bands)
+                ref.check(orc.colourspace(a, dst, src), lambda: pyref.RefImage.from_array(a, orc.SPACES[src]).colourspace(dst, src).numpy(),
+                          (src, dst, bands))
     declined = 0
     for dt in (np.uint8, np.uint16, np.int16, np.int32, np.float32):
         if dt == np.float32:
@@ -241,7 +232,6 @@ def test_oracle_colourspace_wild_floats_and_foreign_formats_match_reference_buil
             a = rng.integers(np.iinfo(dt).min, np.iinfo(dt).max + 1, (19, 21, 4)).astype(dt)
         for src in ALL_SPACES:
             for dst in ALL_SPACES:
-                want = pyref.RefImage.from_array(a, orc.SPACES[src]).colourspace(dst, src).numpy()
                 try:
                     got = orc.colourspace(a, dst, src)
                 except ValueError:
@@ -249,24 +239,23 @@ def test_oracle_colourspace_wild_floats_and_foreign_formats_match_reference_buil
                     assert {src, dst} == {"srgb", "rgb16"} and dt not in (np.uint8, np.uint16), (dt, src, dst)
                     declined += 1
                     continue
-                assert got.dtype == want.dtype and np.array_equal(got, want, equal_nan=True), (dt, src, dst)
+                ref.check(got, lambda: pyref.RefImage.from_array(a, orc.SPACES[src]).colourspace(dst, src).numpy(), (dt, src, dst))
     assert declined == 6
 
 
-@needs_ref
-def test_srgb_rgb16_rows_are_shifting_casts():
+def test_srgb_rgb16_rows_are_shifting_casts(ref):
     """colourspace.c:372, 420: sRGB <-> RGB16 never touch the scRGB tables -- vips_cast(shift) over every band, alpha too:
     up, the bottom bit fills the new byte (cast.c:150-164); down, the high byte"""
     v = np.arange(256, dtype=np.uint8)
     a = np.stack([v, v[::-1], v, v], axis=1).reshape(16, 16, 4)
     up = orc.colourspace(a, "rgb16", "srgb")
     assert np.array_equal(up, (a.astype(np.uint16) << 8) | np.where(a & 1, 255, 0).astype(np.uint16))
-    assert np.array_equal(up, pyref.RefImage.from_array(a, 22).colourspace("rgb16", "srgb").numpy())
-    assert np.array_equal(up, pyref.RefImage.from_array(a, 22).cast(np.uint16, shift=True).numpy())
+    ref.check(up, lambda: pyref.RefImage.from_array(a, 22).colourspace("rgb16", "srgb").numpy())
+    ref.check(up, lambda: pyref.RefImage.from_array(a, 22).cast(np.uint16, shift=True).numpy())
     w = np.arange(65536, dtype=np.uint16).reshape(256, 64, 4)
     down = orc.colourspace(w, "srgb", "rgb16")
     assert np.array_equal(down, (w >> 8).astype(np.uint8))
-    assert np.array_equal(down, pyref.RefImage.from_array(w, 25).colourspace("srgb", "rgb16").numpy())
+    ref.check(down, lambda: pyref.RefImage.from_array(w, 25).colourspace("srgb", "rgb16").numpy())
     L, steps = orc.lib(), (__import__("ctypes").c_int * 8)()
     assert L.orc_colourspace_route(22, 25, steps) == 1 and steps[0] == orc.STEPS["sRGB2RGB16"]
     assert L.orc_colourspace_route(25, 22, steps) == 1 and steps[0] == orc.STEPS["RGB162sRGB"]

@@ -7,8 +7,8 @@ import pytest
 
 from oracle import pyconv, pyref
 from oracle import pyoracle as orc
+from refgold import ref  # noqa: F401
 
-needs_ref = pytest.mark.skipif(not pyref.available(), reason="oracle/_ref not built")
 DTYPES = [np.uint8, np.int8, np.uint16, np.int16, np.uint32, np.int32, np.float32]
 
 # test_convolution.py:43-55
@@ -35,12 +35,12 @@ def same(a, b):
 
 # ------------------------------------------------------------------- CPU
 
-@needs_ref
-def test_gaussmat_matches_reference():
+def test_gaussmat_matches_reference(ref):
     for s, ma, sep, pr in ((0.5, 0.1, True, "integer"), (4.0, 0.2, True, "float"), (1.5, 0.2, False, "integer"),
                            (2.0, 0.2, False, "float"), (0.1, 0.2, True, "integer"), (7.3, 0.05, True, "float")):
-        m1, m2 = pyconv.gaussmat(s, ma, sep, pr), pyconv.ref_gaussmat(s, ma, sep, pr)
-        assert np.array_equal(m1[0], m2[0]) and m1[1] == m2[1] and m1[2] == m2[2]
+        m1 = pyconv.gaussmat(s, ma, sep, pr)
+        ref.check(m1[0], lambda: pyconv.ref_gaussmat(s, ma, sep, pr)[0])
+        ref.check(np.array(m1[1:], np.float64), lambda: np.array(pyconv.ref_gaussmat(s, ma, sep, pr)[1:], np.float64))
 
 
 def test_gaussmat_baseline_mask_is_15_taps():
@@ -51,24 +51,22 @@ def test_gaussmat_baseline_mask_is_15_taps():
     assert m.ravel().tolist() == [3, 20, 3] and scale == 26
 
 
-@needs_ref
 @pytest.mark.parametrize("dt", DTYPES + [np.float64])
-def test_oracle_conv_matches_reference(dt):
+def test_oracle_conv_matches_reference(ref, dt):
     rng = np.random.default_rng(0)
     a = rnd(rng, dt)
     g15 = pyconv.gaussmat(4.0, 0.2, True, "float")
     for m, sc, off in MASKS + [(g15[0], g15[1], 0)]:
         for pr in ("float", "integer"):
-            same(pyconv.ref_conv(a, m, sc, off, pr), pyconv.conv(a, m, sc, off, pr))
+            ref.check(pyconv.conv(a, m, sc, off, pr), lambda: pyconv.ref_conv(a, m, sc, off, pr))
 
 
-@needs_ref
-def test_oracle_conv_vector_semantics_match_reference():
+def test_oracle_conv_vector_semantics_match_reference(ref):
     rng = np.random.default_rng(1)
     a = rnd(rng, np.uint8, (64, 64, 3))
     gi = pyconv.gaussmat(1.2, 0.2, False, "integer")
     for m, sc, off in MASKS + [(gi[0], gi[1], 0)]:
-        same(pyconv.ref_conv(a, m, sc, off, "integer", vector=True), pyconv.conv(a, m, sc, off, "integer", vector=True))
+        ref.check(pyconv.conv(a, m, sc, off, "integer", vector=True), lambda: pyconv.ref_conv(a, m, sc, off, "integer", vector=True))
 
 
 def test_conv_point_values():
@@ -108,12 +106,10 @@ def test_sharpen_identity_when_m1_m2_zero():
     assert np.abs(back - lab).max() < 0.01
 
 
-def test_convsep_mask_orientation_against_reference():
+def test_convsep_mask_orientation_against_reference(ref):
     """convsep.c:92-107 through the reference's own convsep.c / rot.c: an n x 1 mask runs the horizontal
     pass first; a 1 x n mask runs the vertical pass first and then the REVERSED row (vips_rot90), with
     the offset applied in the first pass only.  Asymmetric masks, integer rounding / clipping per pass."""
-    if not pyref.available():
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(21)
     row = np.array([[1.0, 4.0, 9.0, 2.0, -3.0]])
     for dt in (np.uint8, np.int16, np.float32):
@@ -121,31 +117,28 @@ def test_convsep_mask_orientation_against_reference():
         for mask in (row, row.T.copy()):
             for pr in ("float", "integer"):
                 got = pyconv.convsep(a, mask, 13.0, 7.0, pr)
-                want = pyconv.ref_convsep(a, mask, 13.0, 7.0, pr)
-                assert got.dtype == want.dtype and np.array_equal(got, want), (dt, mask.shape, pr)
+                ref.check(got, lambda: pyconv.ref_convsep(a, mask, 13.0, 7.0, pr), (dt, mask.shape, pr))
     # and the orientation matters for these masks: the two orders differ
     assert not np.array_equal(pyconv.convsep(a, row, 13.0, 7.0, "integer"), pyconv.convsep(a, row.T.copy(), 13.0, 7.0, "integer"))
 
 
-def test_sharpen_against_reference_sharpen_c():
+def test_sharpen_against_reference_sharpen_c(ref):
     """The reference's own sharpen.c (build: integer gaussmat at min_ampl 0.1, the LUT, L extraction,
     convsep; generate: sharpen.c:116-168) compiled into oracle/_ref: the oracle must equal it bit for
     bit -- LUT and pixels, several parameter sets, sRGB and LabS inputs, SMALLTILE and FATSTRIP sinks."""
-    if not pyref.available():
-        pytest.skip("oracle/_ref not built")
     for kw in ({}, {"sigma": 1.5, "m2": 5.0, "y2": 20.0}, {"sigma": 0.8, "x1": 1.0, "m1": 0.5, "y3": 5.0}):
         lut_kw = {k: v for k, v in kw.items() if k != "sigma"}
-        assert np.array_equal(pyconv.sharpen_lut(**lut_kw), pyconv.ref_sharpen_lut(**kw)), kw
+        ref.check(pyconv.sharpen_lut(**lut_kw), lambda: pyconv.ref_sharpen_lut(**kw), kw)
     rng = np.random.default_rng(22)
     a = rnd(rng, np.uint8, (150, 170, 3))
     smooth = np.clip(np.add.outer(np.arange(150), np.arange(170))[:, :, None] * 0.7 + rng.integers(0, 12, (150, 170, 3)), 0, 255).astype(np.uint8)
     for img in (a, smooth):
         for kw in ({}, {"sigma": 1.5, "m2": 5.0, "y2": 20.0}, {"sigma": 0.8, "x1": 1.0, "m1": 0.5, "y3": 5.0}):
-            want = pyconv.ref_sharpen(img, "srgb", **kw)
-            assert np.array_equal(pyconv.sharpen(img, "srgb", **kw), want), kw
-            assert np.array_equal(pyconv.ref_sharpen(img, "srgb", tile=(128, 128), **kw), want)  # tile-invariant
+            got = pyconv.sharpen(img, "srgb", **kw)
+            ref.check(got, lambda: pyconv.ref_sharpen(img, "srgb", **kw), kw)
+            ref.check(got, lambda: pyconv.ref_sharpen(img, "srgb", tile=(128, 128), **kw), kw)  # tile-invariant
     labs = orc.colourspace(a, "labs", "srgb")
-    assert np.array_equal(pyconv.sharpen(labs, "labs"), pyconv.ref_sharpen(labs, "labs"))
+    ref.check(pyconv.sharpen(labs, "labs"), lambda: pyconv.ref_sharpen(labs, "labs"))
 
 
 # ------------------------------------------------------------------- GPU

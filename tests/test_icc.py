@@ -20,7 +20,8 @@ from oracle import pylcms
 
 needs_lcms = pytest.mark.skipif(not pylcms.available(), reason="no lcms2 next to Pillow")
 FMT = {np.dtype(np.uint8): 0, np.dtype(np.uint16): 2, np.dtype(np.float32): 6}
-REF_PROFILES = "/root/reference/libvips/colour/profiles"
+# the reference's own profiles (libvips/colour/profiles), copied by tests/golden/make_ref_profiles.py
+REF_PROFILES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "profiles")
 
 
 def host_eval(mode, a, pa, pb=None, depth=8, pcs=0, intent=1):
@@ -188,7 +189,6 @@ def test_v4_lut_profile_against_lcms2(pcs):
 
 
 @needs_lcms
-@pytest.mark.skipif(not os.path.isdir(REF_PROFILES), reason="reference profiles not on this machine")
 def test_reference_profiles_against_lcms2():
     P = lambda n: open(os.path.join(REF_PROFILES, n), "rb").read()
     rng = np.random.default_rng(7)

@@ -6,6 +6,8 @@ import os
 import numpy as np
 import pytest
 
+from refgold import ref  # noqa: F401
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 FIX = np.load(os.path.join(HERE, "golden", "rgba_fixture.npz"))
 
@@ -40,19 +42,16 @@ def test_gpu_linear_thumbnail_parity(vb, oracle, shape, target, bands):
     assert got.shape == want.shape and np.array_equal(got, want)
 
 
-def test_oracle_linear_chain_against_reference_sources():
+def test_oracle_linear_chain_against_reference_sources(ref):
     """CPU: the oracle's linear-light thumbnail against the reference's OWN sources under oracle/_ref --
     premultiply.c, resize.c (shrinkv / reducev / shrinkh / reduceh float branches), unpremultiply.c and the
     sRGB2scRGB / scRGB2sRGB line functions; only the 4th band's trip through vips_colour_build (x 1 / 255,
     x 255, cast) is restated here (colour.c:252-291)."""
     from oracle import pyref
-    if not pyref.available():
-        pytest.skip("oracle/_ref not built")
     from oracle import pyoracle as orc
-    rng = np.random.default_rng(77)
-    for shape, target in (((256, 320, 4), 40), ((200, 150, 3), 33), ((333, 222, 4), 60)):
-        a = rng.integers(0, 256, shape, dtype=np.uint8)
-        h, w, b = shape
+
+    def reference(a, target):
+        h, w, b = a.shape
         hs, vs, _, _ = orc.thumbnail_size(w, h, target)
         lin = pyref.colour_line("sRGB2scRGB", a[:, :, :3]).reshape(h, w, 3)
         if b == 4:
@@ -69,7 +68,11 @@ def test_oracle_linear_chain_against_reference_sources():
         if b == 4:
             al = np.clip((np.float32(255.0) * res[:, :, 3] + np.float32(0)).astype(np.float32).astype(np.float64), 0, 255).astype(np.uint8)
             rgb = np.concatenate([rgb, al[:, :, None]], axis=2)
-        assert np.array_equal(orc.thumbnail_image(a, target, linear=True), rgb), shape
+        return rgb
+    rng = np.random.default_rng(77)
+    for shape, target in (((256, 320, 4), 40), ((200, 150, 3), 33), ((333, 222, 4), 60)):
+        a = rng.integers(0, 256, shape, dtype=np.uint8)
+        ref.check(orc.thumbnail_image(a, target, linear=True), lambda: reference(a, target), shape)
 
 
 @pytest.mark.gpu

@@ -6,8 +6,8 @@ import pytest
 
 from oracle import pyoracle as orc
 from oracle import pyref
+from refgold import ref  # noqa: F401
 
-needs_ref = pytest.mark.skipif(not pyref.available(), reason="oracle/_ref not built")
 DTYPES = [np.uint8, np.int8, np.uint16, np.int16, np.uint32, np.int32, np.float32]
 CASES = [(2.0, None, "lanczos3"), (1.5, None, "cubic"), (1.3, 2.7, "linear"), (2.5, None, "nearest"),
          (3.1, 1.0, "lanczos3"), (1.0, 1.9, "mitchell"), (1.01, None, "linear")]
@@ -21,16 +21,13 @@ def rnd(rng, dt, shape=(40, 57, 3)):
     return rng.integers(i.min, int(i.max) + 1, shape, dtype=np.int64).astype(dt)
 
 
-@needs_ref
 @pytest.mark.parametrize("dt", DTYPES)
-def test_oracle_resize_up_matches_reference(dt):
+def test_oracle_resize_up_matches_reference(ref, dt):
     rng = np.random.default_rng(1)
     a = rnd(rng, dt)
-    x = pyref.RefImage.from_array(a)
     for sc, vs, k in CASES:
-        want = x.resize(sc, vs, kernel=k).numpy()
         got = orc.resize(a, sc, vs, kernel=k)
-        assert want.shape == got.shape and np.array_equal(want, got), (sc, vs, k)
+        ref.check(got, lambda: pyref.RefImage.from_array(a).resize(sc, vs, kernel=k).numpy(), (sc, vs, k))
 
 
 def test_resize_up_geometry_and_edges():

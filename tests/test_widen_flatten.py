@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import pyconv, pyref
+from refgold import ref  # noqa: F401
 
 DTYPES = (np.uint8, np.int8, np.uint16, np.int16, np.uint32, np.int32, np.float32)
 sRGB, RGB16, scRGB = 22, 25, 28
@@ -36,21 +37,20 @@ def cases(rng, shapes):
                     yield a, bg, ma, interp, want
 
 
-@pytest.mark.skipif(not pyref.available(), reason="oracle/_ref not built")
-def test_oracle_flatten_matches_reference():
+def test_oracle_flatten_matches_reference(ref):
     rng = np.random.default_rng(21)
     n = 0
     for a, bg, ma, interp, want in cases(rng, ((9, 13, 2), (7, 12, 4), (5, 6, 5))):
         if want is None:
             continue
-        ref = pyconv.ref_flatten(a, bg, ma, interp)
-        assert ref.dtype == want.dtype and np.array_equal(ref, want), (a.dtype, a.shape, bg, ma, interp)
+        ref.check(want, lambda: pyconv.ref_flatten(a, bg, ma, interp), (a.dtype, a.shape, bg, ma, interp))
         n += 1
     assert n > 400
     a = image(rng, np.uint8, (40, 300, 4))
-    assert np.array_equal(pyconv.ref_flatten(a, (1, 2, 3), tile=(128, 16)), pyconv.flatten(a, (1, 2, 3)))
+    ref.check(pyconv.flatten(a, (1, 2, 3)), lambda: pyconv.ref_flatten(a, (1, 2, 3), tile=(128, 16)))
     one = image(rng, np.uint16, (5, 5, 1))
-    assert np.array_equal(pyconv.ref_flatten(one), one) and np.array_equal(pyconv.flatten(one), one)
+    ref.check(one, lambda: pyconv.ref_flatten(one))
+    assert np.array_equal(pyconv.flatten(one), one)
 
 
 def test_host_twin_matches_oracle():

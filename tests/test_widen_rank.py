@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import pyconv, pyref
+from refgold import ref  # noqa: F401
 
 DTYPES = (np.uint8, np.int8, np.uint16, np.int16, np.uint32, np.int32, np.float32)
 # (width, height, index): median 3x3 / 5x5, min, max, the uchar histogram path (n > 90 and n > 10 mid-index), odd shapes
@@ -23,15 +24,14 @@ def image(rng, dt, shape):
     return a
 
 
-@pytest.mark.skipif(not pyref.available(), reason="oracle/_ref not built")
-def test_oracle_rank_matches_reference():
+def test_oracle_rank_matches_reference(ref):
     rng = np.random.default_rng(11)
     for dt in DTYPES:
         a = image(rng, dt, (37, 45, 3))
         for (rw, rh, idx) in WINDOWS:
-            want = pyconv.ref_rank(a, rw, rh, idx)
-            assert np.array_equal(pyconv.rank(a, rw, rh, idx), want), (dt, rw, rh, idx)
-            assert np.array_equal(pyconv.ref_rank(a, rw, rh, idx, tile=(16, 16)), want)
+            got = pyconv.rank(a, rw, rh, idx)
+            ref.check(got, lambda: pyconv.ref_rank(a, rw, rh, idx), (dt, rw, rh, idx))
+            ref.check(got, lambda: pyconv.ref_rank(a, rw, rh, idx, tile=(16, 16)), (dt, rw, rh, idx))
 
 
 def test_host_twin_matches_oracle():
